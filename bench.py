@@ -20,6 +20,9 @@ What the line reports (N = 1):
                  <= 1e-9, weights, resampling history (count + hash), work counters, every cell of three particles
   cpu_baseline   the oracle's thread pool on this host's cores: logical CPUs, affinity and cgroup quota are printed; the thread count is
                  chosen on steady-state scans; both the best and the all-cores figure are given
+
+--dump-outputs DIR writes, after all timed passes, what the `value` pass's filter holds after its last timed step (see dump_outputs) as
+DIR/<name>.npy.  Scans and seeds are fixed, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -40,6 +43,8 @@ WORLD = "loop"   # 30 m x 30 m room with four pillars, rounded-square loop (BASE
 METRIC = "scans/sec at 256 particles x 1080 beams"
 WORKLOAD = f"PFSlam2D {PARTICLES} particles x {BEAMS} beams, 0.05 m grid, l2_max 0.5, GN+Cauchy(0.15), synthetic 30 m loop room"
 FORCED_GAIN = 0.0008   # meas_sigma_gain of the `resample_forced` regime (default 3: the filter never resamples on this world)
+DUMP_MAP_PARTICLES = 4       # particles whose maps --dump-outputs writes, drawn with a fixed seed from rank 0's shard
+DUMP_BUDGET = 64 << 20       # bytes --dump-outputs may write in all
 
 
 def load_peaks():
@@ -421,7 +426,7 @@ def gpu_arm(args):
     cpu, parity = None, None
     facts = host_facts()
     if world == 1 and not args.no_cpu:
-        cpu_steps = max(4, min(steps, args.cpu_steps))
+        cpu_steps = max(1, min(steps, args.cpu_steps))   # never past scan first + steps: the dataset ends there
         arm, cpu = cpu_measure(ds, facts, first, cpu_steps, first + steps)
         parity = compare(pf_value, arm)
         del arm
@@ -501,6 +506,8 @@ def gpu_arm(args):
             line["parity"] = parity
         if regimes:
             line["regimes"] = regimes
+        if args.dump_outputs:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "bytes": dump_outputs(pf_value, args.dump_outputs, PARTICLES // world)}
         print(json.dumps(line))
     if world > 1:
         import torch.distributed as dist
@@ -539,6 +546,34 @@ def compare(pf, arm):
     return out
 
 
+def dump_outputs(pf, out_dir, local_particles):
+    """Writes what a caller of PFSlam2D receives after the last update as out_dir/<name>.npy: the pose, every particle's state and
+    weights, neff, the best particle and its trajectory (float64), and the occupancy and distance maps of DUMP_MAP_PARTICLES particles
+    drawn with a fixed seed from the first `local_particles` (float32, with their origin cell).  Stops adding maps at DUMP_BUDGET bytes."""
+    st, w = pf.getParticles()
+    best = pf.getBestParticleIdx()
+    arrays = {"pose": pf.getPose(), "particle_states": st, "particle_weights": w, "neff": np.array([pf.getNeff()]),
+              "best_particle": np.array([best], np.float64), "best_trajectory": pf.trajectory(best)}
+    total = sum(a.nbytes for a in arrays.values())
+    sample = np.random.default_rng(0).choice(local_particles, size=min(DUMP_MAP_PARTICLES, local_particles), replace=False)
+    for p in sorted(int(i) for i in sample):
+        maps = {}
+        for kind, export, planes in ((0, pf.exportOccupancy, ("occupied", "visited")), (1, pf.exportDistance, ("sqdist", "valid", "ox", "oy"))):
+            _, mn, mx = pf.mapBounds(p, kind)
+            m = export(p, int(mn[0]), int(mn[1]), int(mx[0] - mn[0]), int(mx[1] - mn[1]))
+            maps[f"map{p:03d}_{'occ' if kind == 0 else 'dm'}_origin"] = mn.astype(np.float64)
+            maps.update({f"map{p:03d}_{k}": m[k].astype(np.float32) for k in planes})
+        size = sum(a.nbytes for a in maps.values())
+        if total + size > DUMP_BUDGET:
+            break
+        arrays.update(maps)
+        total += size
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -553,7 +588,10 @@ def main():
     ap.add_argument("--full-loop", type=int, default=5000, help="scans of the full-loop regime (BASELINE config 4: 5 000)")
     ap.add_argument("--sharded-impl", default="native", choices=["native", "python"])
     ap.add_argument("--prebuild", type=int, default=300, help="untimed scans that build the map before warm-up (both arms)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed filter's state after its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
